@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the Fitch/Sankoff construction pass (BASELINE.json metric: node x column updates / s at 1/2/4/8 B200).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--algo fitch|sankoff] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config NAME] [--algo fitch|sankoff] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (forward + backward + ordered mutation compaction, and for N > 1 the column-range
 gather + merge of the per-rank lists on rank 0) over one batch of synthetic columns. The workload is BASELINE.json
@@ -12,7 +12,8 @@ part of ONE pmb_group (include/panman_b200.h): the library owns the ranges, the 
 NVLink (the packing kernel's stores into peer memory mapped through CUDA IPC), the hand-shakes (stream memory operations)
 and the merge; torch.distributed (NCCL) only all-gathers the 128-byte mailbox handles once and reduces the timings.
 Prints ONE JSON line (rank 0). At N = 1 the line also carries a `configs` table (every BASELINE.json configuration, both
-algorithms where the survey asks for both) measured the same way (CUDA events over 20 pipelined passes).  --impl reference times the reference's own CPU
+algorithms where the survey asks for both) measured the same way (CUDA events over --steps pipelined passes). Every timed
+loop, the end-to-end figures included, runs --steps steps.  --impl reference times the reference's own CPU
 implementation instead.
 """
 import argparse
@@ -48,8 +49,17 @@ def parse():
     ap.add_argument("--no-traffic", action="store_true", help="N = 1: do not measure DRAM traffic with an ncu child run")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the merged lists of the last timed step to DIR/<name>.npy (see dump_outputs); B200 arm only: "
+                         "the reference arm sizes its column sample by a timing probe, so its inputs differ from run to run")
     ap.add_argument("--traffic-child", action="store_true", help=argparse.SUPPRESS)
-    return ap.parse_args()
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs the B200 arm: the reference arm sizes its column sample by a timing probe, "
+                 "so its inputs, and its lists, differ from run to run")
+    return args
 
 
 def workload(args, name=None, algo=None):
@@ -228,6 +238,24 @@ def peak_gbs():
     return 6650.0, "fallback 6650 GB/s (B200_PROFILING.md; MEASURED_PEAKS.json absent)"
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res):
+    """The merged lists a caller of pmb_group_download receives after the last timed step, as out_dir/<name>.npy:
+    node_offsets whole, and the records (pos, type_code) whole when they fit in 64 MB in all, else a fixed seeded sample of
+    them; record_index.npy says which records were kept. Values are exact in float64 (float32 for the 8-bit type codes).
+    The workload is seeded, so the same arguments give the same files on any build that computes the same lists."""
+    off = res.node_offsets.astype(np.float64)
+    n = len(res.pos)
+    k = min(n, (DUMP_BYTES - 4096 - off.nbytes) // 20)  # 4 KB for the .npy headers; record_index, pos f64, type_code f32
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("node_offsets", off), ("record_index", idx.astype(np.float64)), ("pos", res.pos[idx].astype(np.float64)),
+                    ("type_code", res.type_code[idx].astype(np.float32))):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def slice_lists(res, n_nodes, a, b):
     node = np.repeat(np.arange(n_nodes), np.diff(res.node_offsets))
     keep = (res.pos >= a) & (res.pos < b)
@@ -363,6 +391,8 @@ def run_b200_arm(args):
     c0, c1 = pb.column_range(world, C, rank)  # strong scaling: ONE alignment, contiguous tile-aligned ranges
     tree = synth.make_tree(cfg["n_leaves"], cfg["seed"], cfg["kind"])
     N = tree.n_nodes
+    if args.dump_outputs and 8 * (N + 1) > DUMP_BYTES // 2:  # every rank stops here, none waits for the others in a barrier
+        raise SystemExit(f"bench.py: the node offsets of {N} nodes take more than half of the {DUMP_BYTES >> 20} MB of --dump-outputs")
     spec = synth.MsaSpec(cfg["seed"], cfg["p_sub"], cfg["f_gap"], cfg["p_N"])
     codes4, pc = synth.simulate_msa(tree, c0, c1, spec, device=dev)  # this rank's range, generated on its device
     ro = None
@@ -432,6 +462,8 @@ def run_b200_arm(args):
 
     # ---- the result of the last step (outside the timed region): merged lists on rank 0, and the parity check
     res = g.download(copy=True) if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     run_merge_ms = None
     if rank == 0:  # the <= 6 run-merge into NucMut fields follows the gather (outside the timed region; for information)
         nm = g.merge_runs()
@@ -470,7 +502,7 @@ def run_b200_arm(args):
 
         e2e_step()
         barrier()
-        e2e_steps = max(2, min(K, 4))
+        e2e_steps = K
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
             r2 = e2e_step()
@@ -512,7 +544,7 @@ def run_b200_arm(args):
                 same = bool(np.array_equal(r3.node_offsets, res.node_offsets) and np.array_equal(r3.pos, res.pos)
                             and np.array_equal(r3.type_code, res.type_code))
             barrier()
-            runs_steps = max(3, min(K, 10))
+            runs_steps = K
             t0 = time.perf_counter()
             for _ in range(runs_steps):
                 r3 = runs_step()
@@ -586,7 +618,7 @@ def run_b200_arm(args):
             for name, a in (("sars20k", "fitch"), ("indel10k", "fitch"), ("indel10k", "sankoff"), ("caterpillar100k", "fitch"),
                             ("caterpillar100k", "sankoff")):
                 try:
-                    table.append(measure_one(pb, synth, torch, name, a, dev, local, 20, 3))
+                    table.append(measure_one(pb, synth, torch, name, a, dev, local, K, args.warmup))
                 except Exception as e:  # noqa: BLE001
                     table.append({"config": name, "algo": a, "error": str(e)})
             table.append({"config": args.config, "algo": algo, "leaves": cfg["n_leaves"], "nodes": N, "cols": C, "ms": dev_ms_max,
