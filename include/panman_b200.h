@@ -134,7 +134,9 @@ int pmb_set_tree(pmb_ctx* ctx, int32_t n_nodes, int32_t root, const int32_t* chi
  *                   src/panman.cpp:1057-1079, 1583-1604; src/reroot.cpp:189-190).
  * fwd_root_ref    : n_cols or NULL; -1 none, else the forward-pass root reference code (refState,
  *                   src/panman.cpp:1419-1420). Fitch only.
- * col_base        : added to every emitted position (column-range sharding across GPUs). */
+ * col_base        : added to every emitted position (column-range sharding across GPUs). Positions are int32 (the
+ *                   reference's NucMut.nucPosition): 0 <= col_base and col_base + n_cols <= 2^31, else PMB_ERR_INVALID
+ *                   (the same for every upload entry; the group uploads refuse n_cols_total > 2^31). */
 int pmb_run_nuc(pmb_ctx* ctx, int algo, int64_t n_cols, int32_t n_rows, const uint8_t* leaf_codes_4bit,
                 int64_t row_stride_bytes, const uint8_t* leaf_present, const uint8_t* parent_code,
                 const int8_t* root_override, const int8_t* fwd_root_ref, int64_t col_base, int flags,

@@ -664,6 +664,9 @@ static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t
             return fail(c, PMB_ERR_INVALID, "a column range of an encoded batch starts on a multiple of 1024 and ends on one or with the batch");
     }
     if (n_cols > (int64_t(1) << 40)) return fail(c, PMB_ERR_INVALID, "n_cols too large");
+    // positions are int32 (NucMut.nucPosition): every column col_base .. col_base + n_cols - 1 must be one
+    if (col_base < 0 || col_base > (int64_t(1) << 31) - n_cols)
+        return fail(c, PMB_ERR_INVALID, "col_base + n_cols exceeds 2^31 (or col_base < 0): positions are int32");
     PMB_CUDA(cudaSetDevice(c->device));
     // passes still in flight on the backward / compaction streams read what is overwritten here
     PMB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_bwd_done, 0));

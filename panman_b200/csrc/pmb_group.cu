@@ -457,6 +457,9 @@ int pmb_group_connect(pmb_group* g, const void* all_handles) {
     return PMB_OK;
 }
 
+// positions are int32: a column past 2^31 - 1 could not be emitted on any rank
+constexpr int64_t MAX_COLS_TOTAL = int64_t(1) << 31;
+
 // one local rank's range, from a nibble matrix of the range (shard_codes_4bit) or from an encoded batch (runs: the range's
 // columns start at runs_col_begin of it)
 static int upload_shard_impl(pmb_group* g, int local_index, int64_t n_cols_total, int32_t n_rows, const uint8_t* shard_codes_4bit,
@@ -465,6 +468,7 @@ static int upload_shard_impl(pmb_group* g, int local_index, int64_t n_cols_total
                              int64_t runs_col_begin) {
     if (!g || local_index < 0 || local_index >= g->n_local || n_cols_total <= 0) return PMB_ERR_INVALID;
     if (!g->have_tree) return gfail(g, PMB_ERR_NO_TREE, "pmb_group_set_tree has not been called");
+    if (n_cols_total > MAX_COLS_TOTAL) return gfail(g, PMB_ERR_INVALID, "n_cols_total exceeds 2^31: positions are int32");
     if (g->have_input && g->n_cols_total != n_cols_total) {  // a new alignment: every local rank must be given its range again
         for (auto& l : g->local) l.active = false;
         g->have_input = false;
@@ -497,6 +501,7 @@ int pmb_group_upload_shard(pmb_group* g, int local_index, int64_t n_cols_total, 
 int pmb_group_upload_shard_runs(pmb_group* g, int local_index, int64_t n_cols_total, const pmb_runs* shard_runs, const uint8_t* leaf_present,
                                 const uint8_t* shard_parent_code, const int8_t* shard_root_override, const int8_t* shard_fwd_root_ref) {
     if (!g || !shard_runs) return g ? gfail(g, PMB_ERR_INVALID, "null runs") : PMB_ERR_INVALID;
+    if (n_cols_total > MAX_COLS_TOTAL) return gfail(g, PMB_ERR_INVALID, "n_cols_total exceeds 2^31: positions are int32");
     pmb_runs_info info{};
     pmb_runs_describe(shard_runs, &info);
     int64_t b, e;
