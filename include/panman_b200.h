@@ -166,6 +166,22 @@ int pmb_upload_nuc(pmb_ctx* ctx, int64_t n_cols, int32_t n_rows, const uint8_t* 
 int pmb_upload_nuc_async(pmb_ctx* ctx, int64_t n_cols, int32_t n_rows, const uint8_t* leaf_codes_4bit, int64_t row_stride_bytes,
                          const uint8_t* leaf_present, const uint8_t* parent_code, const int8_t* root_override,
                          const int8_t* fwd_root_ref, int64_t col_base);
+/* Leaf codes rebuilt from a PanMAT's mutation lists instead of a code matrix: the upload entry of Tree::reroot (reference
+ * src/reroot.cpp:19-35, getSequenceFromReference). The context's tree (pmb_set_tree) is the tree the pass will run on;
+ * old_* describe the tree the lists were built on, with the same set of leaf rows. Pieces are NucMut fields in HOST memory,
+ * node-major over old node ids: piece_offsets[old_n_nodes + 1], nuc_position, mut_info ((length << 4) + type, type 0..2,
+ * length 1..6), nucs. Positions lie in [0, n_cols). A leaf's code in column c is parent_code[c] overwritten, walking old
+ * root -> leaf, by every piece that covers c, in stored order (NS / NI write their nucs nibble, ND writes '-'): the deepest
+ * node wins, and within a node the later piece. A leaf without pieces of its own gets its nearest ancestor's codes, and every
+ * leaf takes part in the pass (no leaf_present). root_leaf_row >= 0: root_override = that leaf's replayed code in every
+ * column; -1: none. No fwd_root_ref, col_base 0. The replay runs on the device (only the pieces cross the link); afterwards
+ * as pmb_upload_nuc. PMB_ERR_INVALID, before anything is enqueued, for a malformed old tree, leaf rows that differ from the
+ * context's tree, piece_offsets not starting at 0 or not monotone, a type above 2, a length of 0 or above 6, a piece beyond
+ * n_cols, or a root_leaf_row that is not a row. Synchronous: the inputs may be released on return. */
+int pmb_upload_replay(pmb_ctx* ctx, int32_t old_n_nodes, int32_t old_root, const int32_t* old_child_offsets,
+                      const int32_t* old_child_index, const int32_t* old_leaf_row, const int64_t* piece_offsets,
+                      const int32_t* nuc_position, const uint8_t* mut_info, const uint32_t* nucs, int64_t n_cols,
+                      const uint8_t* parent_code, int32_t root_leaf_row);
 int pmb_run_resident(pmb_ctx* ctx, int algo, int flags);
 /* Asynchronous form: enqueues the pass on the context's stream and returns; several passes (and the caller's own
  * stream work ordered with pmb_stream) can be in flight. pmb_wait blocks until the stream drains and reports the

@@ -95,6 +95,14 @@ int pmh_msa_run(pmb_ctx* ctx, pmh_build* b, char* err, size_t err_len);
 /* The same over the GPUs of a box: `group` = a single-process pmb_group (pmb_group_create with all its devices); the columns
  * of the batch are split into contiguous ranges, one per GPU, and the lists come back merged (include/panman_b200.h). */
 int pmh_msa_run_group(pmb_group* group, pmh_build* b, char* err, size_t err_len);
+/* Tree::reroot (reference src/reroot.cpp:4-261) of a built MSA PanMAT, with the tip `leaf_name` as the new root: the tree is
+ * transformed (pmh_tree_reroot); every leaf's sequence is what the build's Node::nucMutation yields for it
+ * (getSequenceFromReference, src/reroot.cpp:19-35), rebuilt on the device by pmb_upload_replay; every column is inferred
+ * again by Fitch (also for a --low-mem-mode build) with the root forced to the tip's own code, and the lists are run-merged
+ * (src/reroot.cpp:134-261). Afterwards pmh_build_tree / _nucmut / _wire / the tuple arrays describe the re-rooted tree (new
+ * node ids); it may be rerooted again. PMB_ERR_INVALID with "Sequence with name ... not found!" for an unknown name, or for a
+ * node that is not a tip (its message from pmh_tree_reroot); PMB_ERR_NO_INPUT before pmh_msa_run / pmh_build_from_msa. */
+int pmh_msa_reroot(pmb_ctx* ctx, pmh_build* b, const char* leaf_name, char* err, size_t err_len);
 int64_t pmh_build_n_cols(const pmh_build* b);
 const uint8_t* pmh_build_codes4(const pmh_build* b, int64_t* row_stride); /* n_leaves rows; NULL once pmh_msa_run consumed it */
 const uint8_t* pmh_build_present(const pmh_build* b);                      /* n_leaves */

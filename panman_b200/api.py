@@ -215,6 +215,21 @@ class Context:
         self._check(self.L.pmb_upload_nuc(self.h, int(n_cols), int(n_rows), _ptr(codes4), int(row_stride), _ptr(leaf_present),
                                           _ptr(parent_code), _ptr(root_override), _ptr(fwd_root_ref), int(col_base)))
 
+    def upload_replay(self, old_tree, piece_offsets, nuc_position, mut_info, nucs, n_cols, parent_code, root_leaf_row=-1):
+        """pmb_upload_replay: the leaf codes of the context's tree rebuilt on the device from a PanMAT's NucMut pieces, built on
+        `old_tree` (n_nodes, root, child_off, child_idx, leaf_row attributes), node-major over its node ids. root_leaf_row >= 0
+        forces the root to that leaf's replayed codes."""
+        co = np.ascontiguousarray(old_tree.child_off, np.int32)
+        ci = np.ascontiguousarray(old_tree.child_idx, np.int32)
+        lr = np.ascontiguousarray(old_tree.leaf_row, np.int32)
+        po = np.ascontiguousarray(piece_offsets, np.int64)
+        pos = np.ascontiguousarray(nuc_position, np.int32)
+        info = np.ascontiguousarray(mut_info, np.uint8)
+        nu = np.ascontiguousarray(nucs, np.uint32)
+        pc = np.ascontiguousarray(parent_code, np.uint8)
+        self._check(self.L.pmb_upload_replay(self.h, int(old_tree.n_nodes), int(old_tree.root), _ptr(co), _ptr(ci), _ptr(lr), _ptr(po),
+                                             _ptr(pos), _ptr(info), _ptr(nu), int(n_cols), _ptr(pc), int(root_leaf_row)))
+
     def run_resident(self, algo=ALGO_FITCH, flags=0) -> Timings:
         self._check(self.L.pmb_run_resident(self.h, int(algo), int(flags)))
         return self.timings()

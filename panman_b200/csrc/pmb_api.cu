@@ -3,6 +3,9 @@
 // There is deliberately no CPU compute path here: without a device every compute call fails.
 #include <cuda_runtime.h>
 
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
+
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -196,6 +199,10 @@ struct pmb_ctx {
     std::vector<int32_t> dfs_rows, h_dfs_slot;
     uint64_t dfs_hash = 0;
     DevBuf d_run_events, d_run_off, d_dfs_slot;
+    // mutation lists replayed into leaf planes (pmb_upload_replay): pieces, records (keys sorted through two buffers, the spare one
+    // then holds the sweep's stacks; code and node per record), events per column, events per (tile, segment) item, CUB scratch
+    DevBuf d_rp_pos, d_rp_info, d_rp_nucs, d_rp_poff, d_rp_pre, d_rp_span, d_rp_nbase, d_rp_roff, d_rp_keys[2], d_rp_code, d_rp_rpre,
+        d_rp_cnt, d_rp_ev[2], d_rp_tmp;
 
     // work + result
     DevBuf d_done, d_fdone, d_ticket, d_block_sums;
@@ -520,7 +527,9 @@ void pmb_destroy(pmb_ctx* c) {
                           &c->d_pos, &c->d_tc, &c->d_states_u8, &c->d_done, &c->d_fdone, &c->d_ticket, &c->d_mcounts, &c->d_moff,
                           &c->d_mpos, &c->d_mtc, &c->d_scan_state, &c->d_trace, &c->d_rm_counts, &c->d_rm_off, &c->d_rm_pos,
                           &c->d_rm_info, &c->d_rm_nucs, &c->d_rm_wire, &c->d_rm_flags, &c->d_rm_oidx, &c->d_col_break, &c->d_merge_err, &c->d_mblock_sums, &c->d_mrel,
-                          &c->d_run_events, &c->d_run_off, &c->d_dfs_slot, &c->d_dir2, &c->d_staging2})
+                          &c->d_run_events, &c->d_run_off, &c->d_dfs_slot, &c->d_dir2, &c->d_staging2, &c->d_rp_pos, &c->d_rp_info,
+                          &c->d_rp_nucs, &c->d_rp_poff, &c->d_rp_pre, &c->d_rp_span, &c->d_rp_roff, &c->d_rp_keys[0], &c->d_rp_keys[1],
+                          &c->d_rp_nbase, &c->d_rp_code, &c->d_rp_rpre, &c->d_rp_cnt, &c->d_rp_ev[0], &c->d_rp_ev[1], &c->d_rp_tmp})
             b->release();
         for (auto& s : c->prog_cache)
             for (DevBuf& b : s.bufs) b.release();
@@ -645,17 +654,211 @@ int pmb_set_tree(pmb_ctx* c, int32_t n_nodes, int32_t root, const int32_t* child
     PMB_GUARDED(c, set_tree_impl(c, n_nodes, root, child_offsets, child_index, leaf_row))
 }
 
-// The leaf codes come either as a nibble matrix (leaf_codes_4bit) or clade-run encoded (runs, columns from runs_col_begin on).
+// pmb_upload_replay's input (host memory) and what its host-side check derives from it
+struct ReplayInput {
+    int32_t n_nodes, root;
+    const int32_t *child_off, *child_idx, *leaf_row;
+    const int64_t* piece_off;
+    const int32_t* pos;
+    const uint8_t* info;
+    const uint32_t* nucs;
+    int32_t root_leaf_row;
+};
+struct ReplayPlan {
+    std::vector<int32_t> pre_of, dfs_rows;  // node -> pre-order index; leaf rows in depth-first order
+    std::vector<int2> span;                 // pre-order index -> [first, end) of its leaves in depth-first order
+    std::vector<int64_t> node_base;         // node -> number of its first record, records numbered pre-order-major
+    int32_t tip_pos = -1;                   // depth-first position of root_leaf_row
+    int64_t n_pieces = 0, n_rec = 0;
+};
+
+// Everything pmb_upload_replay refuses is found here, before anything is enqueued. Returns "" or the reason.
+static std::string replay_check(const ReplayInput& in, int32_t n_rows, int64_t n_cols, ReplayPlan* P) {
+    const int32_t n = in.n_nodes;
+    if (n < 2 || in.root < 0 || in.root >= n || !in.child_off || !in.child_idx || !in.leaf_row || !in.piece_off)
+        return "bad old tree arguments";
+    if (in.child_off[0] != 0 || in.child_off[n] != n - 1) return "old tree: child_offsets must start at 0 and hold n_nodes - 1 children";
+    {
+        std::vector<char> seen(size_t(n), 0);
+        for (int32_t v = 0; v < n; v++) {
+            if (in.child_off[v + 1] < in.child_off[v]) return "old tree: child_offsets not monotone";
+            for (int32_t e = in.child_off[v]; e < in.child_off[v + 1]; e++) {
+                const int32_t ch = in.child_idx[e];
+                if (ch < 0 || ch >= n || ch == in.root || seen[size_t(ch)]) return "old tree: child_index is not a tree";
+                seen[size_t(ch)] = 1;
+            }
+        }
+    }
+    // depth-first walk from the root (children in stored order): pre-order index and leaf interval of every node
+    P->pre_of.assign(size_t(n), -1);
+    P->span.assign(size_t(n), make_int2(0, 0));
+    P->dfs_rows.clear();
+    std::vector<char> row_seen(size_t(n_rows), 0);
+    std::vector<std::pair<int32_t, int32_t>> st;  // (node, next child edge)
+    int32_t n_pre = 0;
+    auto enter = [&](int32_t v) -> bool {
+        const int32_t pre = n_pre++;
+        P->pre_of[size_t(v)] = pre;
+        P->span[size_t(pre)].x = int32_t(P->dfs_rows.size());
+        if (in.child_off[v] == in.child_off[v + 1]) {
+            const int32_t r = in.leaf_row[v];
+            if (r < 0 || r >= n_rows || row_seen[size_t(r)]) return false;
+            row_seen[size_t(r)] = 1;
+            P->dfs_rows.push_back(r);
+            P->span[size_t(pre)].y = int32_t(P->dfs_rows.size());
+        } else {
+            if (in.leaf_row[v] != -1) return false;
+            st.emplace_back(v, in.child_off[v]);
+        }
+        return true;
+    };
+    if (in.child_off[in.root] == in.child_off[in.root + 1]) return "old tree: the root must be an internal node";
+    enter(in.root);
+    while (!st.empty()) {
+        auto& f = st.back();
+        if (f.second < in.child_off[f.first + 1]) {
+            if (!enter(in.child_idx[f.second++])) return "old tree: its leaf rows are not the rows of the tree set on the context";
+        } else {
+            P->span[size_t(P->pre_of[size_t(f.first)])].y = int32_t(P->dfs_rows.size());
+            st.pop_back();
+        }
+    }
+    if (n_pre != n) return "old tree: not connected";
+    if (int32_t(P->dfs_rows.size()) != n_rows) return "old tree: its leaf rows are not the rows of the tree set on the context";
+    if (in.root_leaf_row < -1 || in.root_leaf_row >= n_rows) return "root_leaf_row is not a row of the tree";
+    P->tip_pos = -1;
+    for (int32_t i = 0; i < n_rows && in.root_leaf_row >= 0; i++)
+        if (P->dfs_rows[size_t(i)] == in.root_leaf_row) P->tip_pos = i;
+    // pieces: NucMut fields, node-major
+    if (in.piece_off[0] != 0) return "piece_offsets must start at 0";
+    for (int32_t v = 0; v < n; v++)
+        if (in.piece_off[v + 1] < in.piece_off[v]) return "piece_offsets not monotone";
+    P->n_pieces = in.piece_off[n];
+    if (P->n_pieces > 0 && (!in.pos || !in.info || !in.nucs)) return "null piece arrays";
+    std::vector<int64_t> by_pre(size_t(n), 0);  // records per node, at its pre-order index
+    for (int32_t v = 0; v < n; v++)
+        for (int64_t k = in.piece_off[v]; k < in.piece_off[v + 1]; k++) {
+            const int type = in.info[k] & 15, len = in.info[k] >> 4;
+            if (type > 2) return "piece " + std::to_string(k) + ": type " + std::to_string(type) + " (only NS 0, ND 1, NI 2)";
+            if (len < 1 || len > 6) return "piece " + std::to_string(k) + ": length " + std::to_string(len) + " (1 .. 6)";
+            if (in.pos[k] < 0 || int64_t(in.pos[k]) + len > n_cols) return "piece " + std::to_string(k) + ": positions beyond n_cols";
+            by_pre[size_t(P->pre_of[size_t(v)])] += len;
+        }
+    P->n_rec = 0;
+    for (int64_t& x : by_pre) {
+        const int64_t cnt = x;
+        x = P->n_rec;
+        P->n_rec += cnt;
+    }
+    if (P->n_rec >= (int64_t(1) << 32)) return "more than 2^32 piece positions";
+    P->node_base.resize(size_t(n));
+    for (int32_t v = 0; v < n; v++) P->node_base[size_t(v)] = by_pre[size_t(P->pre_of[size_t(v)])];
+    return "";
+}
+
+extern "C++" {
+template <class F>
+static int with_cub_scratch(pmb_ctx* c, F f) {  // f(temp, bytes): a CUB device call, sized first
+    size_t bytes = 0;
+    PMB_CUDA(f(nullptr, bytes));
+    PMB_CUDA(c->d_rp_tmp.ensure(std::max<size_t>(bytes, 16)));
+    PMB_CUDA(f(c->d_rp_tmp.p, bytes));
+    return PMB_OK;
+}
+}
+
+static unsigned blocks_for(long long n) { return unsigned(std::max<long long>(1, (n + 255) / 256)); }
+
+// Replay kernels on c->stream: pieces -> sorted records -> per-column sweep (counted, then written) -> events sorted into
+// (tile, segment) items in c->d_run_events / c->d_run_off, the layout expand_runs_kernel reads. d_parent: the parent codes on
+// the device; d_tip (or NULL): receives the code of the leaf at P.tip_pos in every column.
+static int replay_events(pmb_ctx* c, const ReplayInput& in, const ReplayPlan& P, int64_t n_cols, int32_t n_rows, int32_t n_seg,
+                         int32_t seg_rows, const uint8_t* d_parent, int8_t* d_tip) {
+    cudaStream_t s = c->stream;
+    const int32_t n = in.n_nodes;
+    const long long NP = P.n_pieces, R = P.n_rec;
+    int rec_bits = 1, col_bits = 1;
+    while ((1LL << rec_bits) < R) rec_bits++;
+    while ((1LL << col_bits) <= n_cols) col_bits++;  // column + 1 <= n_cols < 2^31: rec_bits + col_bits <= 64
+    PMB_CUDA(c->d_rp_poff.ensure(size_t(n + 1) * sizeof(long long)));
+    PMB_CUDA(c->d_rp_pre.ensure(size_t(n) * sizeof(int)));
+    PMB_CUDA(c->d_rp_span.ensure(size_t(n) * sizeof(int2)));
+    PMB_CUDA(c->d_rp_nbase.ensure(size_t(n) * sizeof(long long)));
+    PMB_CUDA(cudaMemcpyAsync(c->d_rp_poff.p, in.piece_off, size_t(n + 1) * sizeof(long long), cudaMemcpyHostToDevice, s));
+    PMB_CUDA(cudaMemcpyAsync(c->d_rp_pre.p, P.pre_of.data(), size_t(n) * sizeof(int), cudaMemcpyHostToDevice, s));
+    PMB_CUDA(cudaMemcpyAsync(c->d_rp_span.p, P.span.data(), size_t(n) * sizeof(int2), cudaMemcpyHostToDevice, s));
+    PMB_CUDA(cudaMemcpyAsync(c->d_rp_nbase.p, P.node_base.data(), size_t(n) * sizeof(long long), cudaMemcpyHostToDevice, s));
+    PMB_CUDA(c->d_rp_cnt.ensure(size_t(std::max<long long>(NP, n_cols + 1)) * sizeof(long long)));
+    PMB_CUDA(c->d_rp_roff.ensure(size_t(std::max<long long>(NP, n_cols + 1)) * sizeof(long long)));
+    for (int k = 0; k < 2; k++) PMB_CUDA(c->d_rp_keys[k].ensure(size_t(std::max<long long>(R, 2)) * sizeof(unsigned long long)));
+    PMB_CUDA(c->d_rp_code.ensure(size_t(std::max<long long>(R, 16))));
+    PMB_CUDA(c->d_rp_rpre.ensure(size_t(std::max<long long>(R, 4)) * sizeof(int)));
+    cub::DoubleBuffer<unsigned long long> keys(c->d_rp_keys[0].as<unsigned long long>(), c->d_rp_keys[1].as<unsigned long long>());
+    int rc;
+    if (NP > 0) {
+        PMB_CUDA(c->d_rp_pos.ensure(size_t(NP) * sizeof(int32_t)));
+        PMB_CUDA(c->d_rp_info.ensure(size_t(NP)));
+        PMB_CUDA(c->d_rp_nucs.ensure(size_t(NP) * sizeof(uint32_t)));
+        PMB_CUDA(cudaMemcpyAsync(c->d_rp_pos.p, in.pos, size_t(NP) * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        PMB_CUDA(cudaMemcpyAsync(c->d_rp_info.p, in.info, size_t(NP), cudaMemcpyHostToDevice, s));
+        PMB_CUDA(cudaMemcpyAsync(c->d_rp_nucs.p, in.nucs, size_t(NP) * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+        long long* len = c->d_rp_cnt.as<long long>();
+        long long* roff = c->d_rp_roff.as<long long>();
+        replay_piece_len_kernel<<<blocks_for(NP), 256, 0, s>>>(c->d_rp_info.as<uint8_t>(), NP, len);
+        if ((rc = with_cub_scratch(c, [&](void* t, size_t& b) { return cub::DeviceScan::ExclusiveSum(t, b, len, roff, NP, s); }))) return rc;
+        replay_records_kernel<<<blocks_for(NP), 256, 0, s>>>(c->d_rp_poff.as<long long>(), n, c->d_rp_nbase.as<long long>(), c->d_rp_pre.as<int>(),
+                                                             c->d_rp_pos.as<int32_t>(), c->d_rp_info.as<uint8_t>(), c->d_rp_nucs.as<uint32_t>(), NP,
+                                                             roff, rec_bits, keys.Current(), c->d_rp_code.as<uint8_t>(), c->d_rp_rpre.as<int>());
+        PMB_CUDA(cudaGetLastError());
+        if ((rc = with_cub_scratch(c, [&](void* t, size_t& b) {
+                 return cub::DeviceRadixSort::SortKeys(t, b, keys, R, 0, rec_bits + col_bits, s);
+             })))
+            return rc;
+    }
+    // count the events of every column, offsets by an exclusive scan over n_cols + 1 counts (the last one 0: the total)
+    long long* cnt = c->d_rp_cnt.as<long long>();
+    long long* ev_off = c->d_rp_roff.as<long long>();
+    PMB_CUDA(cudaMemsetAsync(cnt + n_cols, 0, sizeof(long long), s));
+    replay_sweep_kernel<false><<<blocks_for(n_cols), 256, 0, s>>>(keys.Current(), c->d_rp_code.as<uint8_t>(), c->d_rp_rpre.as<int>(), R, rec_bits, c->d_rp_span.as<int2>(), d_parent,
+                                                                  n_cols, n_rows, n_seg, seg_rows, P.tip_pos, keys.Alternate(), cnt,
+                                                                  nullptr, nullptr, nullptr);
+    PMB_CUDA(cudaGetLastError());
+    if ((rc = with_cub_scratch(c, [&](void* t, size_t& b) { return cub::DeviceScan::ExclusiveSum(t, b, cnt, ev_off, n_cols + 1, s); })))
+        return rc;
+    long long E = 0;
+    PMB_CUDA(cudaMemcpyAsync(&E, ev_off + n_cols, sizeof(long long), cudaMemcpyDeviceToHost, s));
+    PMB_CUDA(cudaStreamSynchronize(s));
+    for (int k = 0; k < 2; k++) PMB_CUDA(c->d_rp_ev[k].ensure(size_t(std::max<long long>(E, 2)) * sizeof(unsigned long long)));
+    cub::DoubleBuffer<unsigned long long> ev(c->d_rp_ev[0].as<unsigned long long>(), c->d_rp_ev[1].as<unsigned long long>());
+    replay_sweep_kernel<true><<<blocks_for(n_cols), 256, 0, s>>>(keys.Current(), c->d_rp_code.as<uint8_t>(), c->d_rp_rpre.as<int>(), R, rec_bits, c->d_rp_span.as<int2>(), d_parent,
+                                                                 n_cols, n_rows, n_seg, seg_rows, P.tip_pos, keys.Alternate(), nullptr, ev_off,
+                                                                 ev.Current(), d_tip);
+    PMB_CUDA(cudaGetLastError());
+    const long long n_items = (long long)c->T * n_seg;
+    int item_bits = 1;
+    while ((1LL << item_bits) <= n_items) item_bits++;
+    if (E > 0 && (rc = with_cub_scratch(c, [&](void* t, size_t& b) { return cub::DeviceRadixSort::SortKeys(t, b, ev, E, 0, 32 + item_bits, s); })))
+        return rc;
+    PMB_CUDA(c->d_run_events.ensure(size_t(std::max<long long>(E, 4)) * sizeof(uint32_t)));
+    PMB_CUDA(c->d_run_off.ensure(size_t(n_items + 1) * sizeof(long long)));
+    replay_items_kernel<<<blocks_for(std::max(E, n_items + 1)), 256, 0, s>>>(ev.Current(), E, n_items, c->d_run_events.as<uint32_t>(),
+                                                                            c->d_run_off.as<long long>());
+    PMB_CUDA(cudaGetLastError());
+    return PMB_OK;
+}
+
+// The leaf codes come either as a nibble matrix (leaf_codes_4bit), clade-run encoded (runs, columns from runs_col_begin on) or
+// as the mutation lists of a PanMAT replayed over parent_code (replay).
 static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t* leaf_codes_4bit, int64_t row_stride_bytes,
                        const uint8_t* leaf_present, const uint8_t* parent_code, const int8_t* root_override,
                        const int8_t* fwd_root_ref, int64_t col_base, bool sync, const pmb_runs* runs = nullptr,
-                       int64_t runs_col_begin = 0) {
+                       int64_t runs_col_begin = 0, const ReplayInput* replay = nullptr) {
     if (!c) return PMB_ERR_INVALID;
     if (!c->stream) return fail(c, PMB_ERR_CUDA, "no usable CUDA device; there is no CPU fallback");
     if (!c->have_tree) return fail(c, PMB_ERR_NO_TREE, "pmb_set_tree has not been called");
-    if (n_cols <= 0 || (!leaf_codes_4bit && !runs) || !parent_code) return fail(c, PMB_ERR_INVALID, "bad input arguments");
+    if (n_cols <= 0 || (!leaf_codes_4bit && !runs && !replay) || !parent_code) return fail(c, PMB_ERR_INVALID, "bad input arguments");
     if (n_rows != c->prog.n_rows) return fail(c, PMB_ERR_INVALID, "n_rows does not match the tree's leaf count");
-    if (!runs && row_stride_bytes < (n_cols + 1) / 2) return fail(c, PMB_ERR_INVALID, "row_stride_bytes too small");
+    if (!runs && !replay && row_stride_bytes < (n_cols + 1) / 2) return fail(c, PMB_ERR_INVALID, "row_stride_bytes too small");
     if (runs) {
         if (runs->order_hash != c->dfs_hash || runs->n_rows != n_rows)
             return fail(c, PMB_ERR_INVALID, "the batch was encoded for another tree (leaf order differs)");
@@ -667,6 +870,11 @@ static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t
     // positions are int32 (NucMut.nucPosition): every column col_base .. col_base + n_cols - 1 must be one
     if (col_base < 0 || col_base > (int64_t(1) << 31) - n_cols)
         return fail(c, PMB_ERR_INVALID, "col_base + n_cols exceeds 2^31 (or col_base < 0): positions are int32");
+    ReplayPlan plan;
+    if (replay) {
+        const std::string e = replay_check(*replay, n_rows, n_cols, &plan);
+        if (!e.empty()) return fail(c, PMB_ERR_INVALID, e);
+    }
     PMB_CUDA(cudaSetDevice(c->device));
     // passes still in flight on the backward / compaction streams read what is overwritten here
     PMB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_bwd_done, 0));
@@ -693,6 +901,14 @@ static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t
     PMB_CUDA(cudaMemcpyAsync(t, parent_code, size_t(n_cols), cudaMemcpyDefault, c->stream));
     if (root_override) PMB_CUDA(cudaMemcpyAsync(t + n_cols, root_override, size_t(n_cols), cudaMemcpyDefault, c->stream));
     if (fwd_root_ref) PMB_CUDA(cudaMemcpyAsync(t + 2 * n_cols, fwd_root_ref, size_t(n_cols), cudaMemcpyDefault, c->stream));
+    int32_t rp_seg = 0, rp_seg_rows = 0;
+    if (replay) {  // the tip's replayed codes become the root override
+        runs_segments(n_rows, c->T, &rp_seg, &rp_seg_rows);
+        const bool tip = replay->root_leaf_row >= 0;
+        if ((rc = replay_events(c, *replay, plan, n_cols, n_rows, rp_seg, rp_seg_rows, t, tip ? reinterpret_cast<int8_t*>(t + n_cols) : nullptr)))
+            return rc;
+        if (tip) root_override = reinterpret_cast<const int8_t*>(t + n_cols);
+    }
     PMB_CUDA(c->d_colparams.ensure(size_t(c->T) * 128 * sizeof(uint4)));
     {
         long long threads = (long long)c->T * 32 * 32;
@@ -710,7 +926,7 @@ static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t
     // speed of the PCIe copy alone (measured on B200: the kernel reading pinned memory in place reaches 47 GB/s, the copy
     // engine 54 GB/s; tools/e2e_breakdown.py). Pageable memory takes the same path at the driver's staging speed.
     bool on_device = false;
-    if (!runs) {
+    if (!runs && !replay) {
         cudaPointerAttributes attr{};
         if (cudaPointerGetAttributes(&attr, leaf_codes_4bit) == cudaSuccess)
             on_device = attr.type == cudaMemoryTypeDevice || attr.type == cudaMemoryTypeManaged;
@@ -759,6 +975,15 @@ static int upload_impl(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8_t
         }
         PMB_CUDA(cudaEventRecord(c->ev_fork, copy));  // a later upload's copies into these buffers are ordered behind c->stream anyway;
         PMB_CUDA(cudaStreamWaitEvent(c->stream, c->ev_fork, 0));  // this joins the copy stream so that a wait on c->stream covers it
+    } else if (replay) {
+        PMB_CUDA(c->d_dfs_slot.ensure(size_t(n_rows) * sizeof(int)));
+        c->h_dfs_slot.resize(size_t(n_rows));
+        for (int32_t i = 0; i < n_rows; i++) c->h_dfs_slot[size_t(i)] = c->prog.row_slot[size_t(plan.dfs_rows[size_t(i)])];
+        PMB_CUDA(cudaMemcpyAsync(c->d_dfs_slot.p, c->h_dfs_slot.data(), size_t(n_rows) * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        const long long n_items = (long long)c->T * rp_seg;
+        expand_runs_kernel<<<blocks_for(n_items * 32), 256, 0, c->stream>>>(c->d_run_events.as<uint32_t>(), c->d_run_off.as<long long>(), 0, 0, n_items,
+                                                                            rp_seg, rp_seg_rows, n_rows, c->d_dfs_slot.as<int>(),
+                                                                            c->d_colparams.as<uint4>(), c->d_leaf_planes.as<uint4>());
     } else if (on_device) {
         pack(leaf_codes_4bit, row_stride_bytes, 0, n_rows);
     } else {
@@ -823,6 +1048,16 @@ int pmb_upload_nuc_async(pmb_ctx* c, int64_t n_cols, int32_t n_rows, const uint8
                          const int8_t* fwd_root_ref, int64_t col_base) {
     PMB_GUARDED(c, upload_impl(c, n_cols, n_rows, leaf_codes_4bit, row_stride_bytes, leaf_present, parent_code, root_override,
                                fwd_root_ref, col_base, false))
+}
+
+int pmb_upload_replay(pmb_ctx* c, int32_t old_n_nodes, int32_t old_root, const int32_t* old_child_offsets, const int32_t* old_child_index,
+                      const int32_t* old_leaf_row, const int64_t* piece_offsets, const int32_t* nuc_position, const uint8_t* mut_info,
+                      const uint32_t* nucs, int64_t n_cols, const uint8_t* parent_code, int32_t root_leaf_row) {
+    if (!c) return PMB_ERR_INVALID;
+    const ReplayInput in{old_n_nodes, old_root, old_child_offsets, old_child_index, old_leaf_row, piece_offsets, nuc_position, mut_info, nucs,
+                         root_leaf_row};
+    PMB_GUARDED(c, upload_impl(c, n_cols, c->have_tree ? c->prog.n_rows : 0, nullptr, 0, nullptr, parent_code, nullptr, nullptr, 0, true,
+                               nullptr, 0, &in))
 }
 
 static int run_impl(pmb_ctx* c, int algo, int flags, bool async) {

@@ -2062,6 +2062,124 @@ expand_runs_kernel(const uint32_t* events, const long long* item_off, long long 
     }
 }
 
+// ---- a PanMAT's mutation lists -> the clade-run events expand_runs_kernel turns into leaf planes (pmb_upload_replay) ----
+// Every piece position becomes a record. Records are numbered by the pre-order index of their node in the tree the lists were
+// built on, then in stored order within the node, and sorted by column << rec_bits | record number: per column, the nodes of
+// the records are then nested intervals of that tree's depth-first leaf order, and a leaf's code is the code of the last
+// record whose interval holds it (the deepest node wins, and within a node the later piece).
+
+__device__ __forceinline__ long long lower_bound_u64(const unsigned long long* a, long long n, unsigned long long key) {
+    long long lo = 0, hi = n;
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        if (a[mid] < key) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void replay_piece_len_kernel(const uint8_t* mut_info, long long n_pieces, long long* len) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_pieces) len[i] = mut_info[i] >> 4;
+}
+
+// one thread per piece. rec_off: exclusive scan of the piece lengths (node-major); node_base[v]: number of node v's first record
+// (pre-order-major). A deletion writes '-' whatever its nucs hold.
+__global__ void replay_records_kernel(const long long* piece_off, int n_nodes, const long long* node_base, const int* pre_of,
+                                      const int32_t* nuc_position, const uint8_t* mut_info, const uint32_t* nucs, long long n_pieces,
+                                      const long long* rec_off, int rec_bits, unsigned long long* keys, uint8_t* rec_code, int* rec_pre) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pieces) return;
+    int lo = 0, hi = n_nodes - 1;  // the node owning piece i: the last v with piece_off[v] <= i
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (piece_off[mid] <= i) lo = mid;
+        else hi = mid - 1;
+    }
+    const int len = mut_info[i] >> 4, type = mut_info[i] & 15, pre = pre_of[lo];
+    const unsigned long long col = (unsigned long long)nuc_position[i];
+    const uint32_t nu = nucs[i];
+    const long long r = node_base[lo] + rec_off[i] - rec_off[piece_off[lo]];
+    for (int j = 0; j < len; j++) {
+        keys[r + j] = ((col + j) << rec_bits) | (unsigned long long)(r + j);
+        rec_code[r + j] = type == 1 ? uint8_t(0) : uint8_t((nu >> (4 * (5 - j))) & 15u);
+        rec_pre[r + j] = pre;
+    }
+}
+
+// One thread per column sweeps its sorted records with a stack of open intervals (kept in stack_mem at the column's own
+// record range, so it can never overflow) and emits an event wherever the code seen by expand_runs_kernel changes along the
+// leaf order: at a change of the leaf code, and at the first leaf of every segment whose code is not the parent code (each
+// (tile, segment) item restarts from the parent planes). Events of one (leaf, column) compose by XOR. EMIT = false only
+// counts them; EMIT = true writes item << 32 | event (pmb_runs.h layout) and the code of the leaf at tip_pos.
+template <bool EMIT>
+__global__ void replay_sweep_kernel(const unsigned long long* keys, const uint8_t* rec_code, const int* rec_pre, long long n_rec, int rec_bits, const int2* span,
+                                    const uint8_t* parent_code, long long n_cols, int n_rows, int n_seg, int seg_rows, int tip_pos,
+                                    unsigned long long* stack_mem, long long* counts, const long long* ev_off, unsigned long long* ev_out,
+                                    int8_t* tip_code) {
+    const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n_cols) return;
+    const long long a = lower_bound_u64(keys, n_rec, (unsigned long long)c << rec_bits);
+    const long long b = lower_bound_u64(keys, n_rec, (unsigned long long)(c + 1) << rec_bits);
+    const unsigned long long rec_mask = (1ull << rec_bits) - 1;
+    const int pc = parent_code[c] & 15;
+    const unsigned long long item0 = (unsigned long long)(c / TILE_COLS) * n_seg;
+    const uint32_t col_field = uint32_t(c % TILE_COLS) << 4;
+    unsigned long long* out = EMIT ? ev_out + ev_off[c] : nullptr;
+    long long n_ev = 0, next_seg = seg_rows;
+    int val = pc, tipv = pc;  // val: the code expand_runs_kernel holds at the current leaf
+    auto emit = [&](long long p, int x) {
+        if (EMIT) {
+            const long long seg = p / seg_rows;
+            out[n_ev] = ((item0 + seg) << 32) | (uint32_t(p - seg * seg_rows) << 14) | col_field | uint32_t(x);
+        }
+        n_ev++;
+    };
+    auto change = [&](long long p, int nv) {  // from leaf p on, the code is nv (p never decreases)
+        if (p >= n_rows) return;
+        for (; next_seg <= p; next_seg += seg_rows) {
+            if (next_seg < p) {
+                if (val != pc) emit(next_seg, val ^ pc);
+            } else {
+                val = pc;
+            }
+        }
+        if (nv != val) {
+            emit(p, nv ^ val);
+            val = nv;
+        }
+        if (p <= tip_pos) tipv = nv;
+    };
+    unsigned long long* st = stack_mem + a;  // (interval end << 4) | code
+    long long sp = 0;
+    for (long long r = a; r < b; r++) {
+        const long long k = (long long)(keys[r] & rec_mask);
+        const int2 s = span[rec_pre[k]];
+        const int code = rec_code[k];
+        while (sp > 0 && (long long)(st[sp - 1] >> 4) <= s.x) {
+            const long long end = (long long)(st[--sp] >> 4);
+            change(end, sp ? int(st[sp - 1] & 15) : pc);
+        }
+        change(s.x, code);
+        st[sp++] = ((unsigned long long)s.y << 4) | (unsigned long long)code;
+    }
+    while (sp > 0) {
+        const long long end = (long long)(st[--sp] >> 4);
+        change(end, sp ? int(st[sp - 1] & 15) : pc);
+    }
+    for (; next_seg < n_rows; next_seg += seg_rows)
+        if (val != pc) emit(next_seg, val ^ pc);
+    if (!EMIT) counts[c] = n_ev;
+    else if (tip_code) tip_code[c] = int8_t(tipv);
+}
+
+// sorted item << 32 | event keys -> the events and item offsets expand_runs_kernel reads
+__global__ void replay_items_kernel(const unsigned long long* ev, long long n_ev, long long n_items, uint32_t* ev32, long long* item_off) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_ev) ev32[i] = uint32_t(ev[i]);
+    if (i <= n_items) item_off[i] = lower_bound_u64(ev, n_ev, (unsigned long long)i << 32);
+}
+
 // per-column parameters -> planes; one warp per 32-column group (ballot builds the planes)
 __global__ void pack_colparams_kernel(const uint8_t* parent_code, const int8_t* root_override, const int8_t* fwd_root_ref,
                                       long long n_cols, int T, uint4* colparams) {

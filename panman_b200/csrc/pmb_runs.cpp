@@ -47,6 +47,17 @@ uint64_t leaf_order_hash(const std::vector<int32_t>& rows) {
     return h ^ (uint64_t(rows.size()) << 32);
 }
 
+// enough (tile, segment) items to give every resident warp of the device one, never fewer than 64 leaves per segment (every
+// segment start re-states its first leaf in full), never more than the row field holds
+void runs_segments(int64_t n_rows, int64_t T, int32_t* n_seg_out, int32_t* seg_rows_out) {
+    int64_t n_seg = std::max<int64_t>(1, (8192 + T - 1) / T);
+    n_seg = std::min<int64_t>(n_seg, std::max<int64_t>(1, n_rows / 64));
+    n_seg = std::max<int64_t>(n_seg, (n_rows + RUNS_MAX_SEG_ROWS - 1) / RUNS_MAX_SEG_ROWS);
+    const int64_t seg_rows = (n_rows + n_seg - 1) / n_seg;
+    *n_seg_out = int32_t((n_rows + seg_rows - 1) / seg_rows);
+    *seg_rows_out = int32_t(seg_rows);
+}
+
 }  // namespace pmb
 
 namespace {
@@ -111,13 +122,9 @@ int pmb_runs_encode(int32_t n_nodes, int32_t root, const int32_t* child_offsets,
         }
         const int64_t T = (n_cols + 1023) / 1024;
         if (T > (int64_t(1) << 30)) return PMB_ERR_INVALID;
-        // segments: enough (tile, segment) items to give every resident warp of the device one, never fewer than 64 leaves
-        // per segment (every segment start re-states its first leaf in full), never more than the row field holds
-        int64_t n_seg = std::max<int64_t>(1, (8192 + T - 1) / T);
-        n_seg = std::min<int64_t>(n_seg, std::max<int64_t>(1, n_rows / 64));
-        n_seg = std::max<int64_t>(n_seg, (int64_t(n_rows) + pmb::RUNS_MAX_SEG_ROWS - 1) / pmb::RUNS_MAX_SEG_ROWS);
-        const int64_t seg_rows = (int64_t(n_rows) + n_seg - 1) / n_seg;
-        n_seg = (int64_t(n_rows) + seg_rows - 1) / seg_rows;
+        int32_t n_seg32 = 0, seg_rows32 = 0;
+        pmb::runs_segments(n_rows, T, &n_seg32, &seg_rows32);
+        const int64_t n_seg = n_seg32, seg_rows = seg_rows32;
 
         R = new pmb_runs();
         R->n_cols = n_cols;

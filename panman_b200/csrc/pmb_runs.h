@@ -31,4 +31,6 @@ constexpr uint32_t RUNS_MAX_SEG_ROWS = (1u << 18) - 2;
 std::vector<int32_t> dfs_leaf_rows(int32_t n_nodes, int32_t root, const int32_t* child_off, const int32_t* child_idx,
                                    const int32_t* leaf_row);
 uint64_t leaf_order_hash(const std::vector<int32_t>& rows);
+// leaves per (tile, segment) item for n_rows leaves and T column tiles (pmb_runs_encode, pmb_upload_replay)
+void runs_segments(int64_t n_rows, int64_t T, int32_t* n_seg, int32_t* seg_rows);
 }  // namespace pmb

@@ -140,13 +140,15 @@ def reroot_newick(newick: str, leaf_name: str) -> HostTree:
 
 
 class MsaBuild:
-    """panmanUtils -M msa.fa -N tree.nwk [--reference id] [--low-mem-mode] through libpanman_b200."""
+    """panmanUtils -M msa.fa -N tree.nwk [--reference id] [--low-mem-mode] through libpanman_b200. The build keeps its handle
+    until close(): reroot() works on it."""
 
     def __init__(self, ctx, fasta: bytes, newick: str, reference: str = "", low_mem_mode: bool = False):
         """ctx: a Context (one GPU) or a single-process Group (pmh_msa_run_group: column ranges over the GPUs of the box)."""
         from .api import Group
 
         L = load_host_library()
+        self.L = L
         err = C.create_string_buffer(512)
         if isinstance(ctx, Group):
             vp = C.c_void_p
@@ -161,10 +163,16 @@ class MsaBuild:
             h = L.pmh_build_from_msa(ctx.h, fasta, len(fasta), newick.encode(), reference.encode(), int(low_mem_mode), err, 512)
         if not h:
             raise RuntimeError(err.value.decode())
-        self.tree = HostTree(L.pmh_build_tree(h), owned=False)
+        self.h = h
         n = C.c_int64()
         p = L.pmh_build_consensus(h, C.byref(n))
         self.consensus = C.string_at(p, n.value)
+        self._refresh()
+
+    def _refresh(self):
+        """tree, nucmut, wire, tuple arrays and seconds from the handle (after the build and after every reroot)."""
+        L, h = self.L, self.h
+        self.tree = HostTree(L.pmh_build_tree(h), owned=False)
         self.nucmut = []
         for v in range(self.tree.n_nodes):
             k = L.pmh_build_n_nucmut(h, v)
@@ -178,7 +186,34 @@ class MsaBuild:
         self.tuple_pos = np.ctypeslib.as_array(L.pmh_build_tuple_pos(h), (max(nt, 1),))[:nt].copy()
         self.tuple_type_code = np.ctypeslib.as_array(L.pmh_build_tuple_type_code(h), (max(nt, 1),))[:nt].copy()
         self.seconds = list(np.ctypeslib.as_array(L.pmh_build_seconds(h), (4,)))
-        L.pmh_build_free(h)
+
+    def reroot(self, ctx, leaf_name: str):
+        """Tree::reroot (reference src/reroot.cpp) on the built PanMAT (pmh_msa_reroot), on one GPU: the mutation lists are
+        replayed into the leaf sequences on the device and every column is inferred again on the re-rooted tree. The
+        attributes then describe the re-rooted tree."""
+        from .api import Context, PanmanError
+
+        if not isinstance(ctx, Context):
+            raise TypeError("reroot runs on one GPU: pass a Context")
+        if not self.h:
+            raise RuntimeError("the build was closed")
+        self.L.pmh_msa_reroot.argtypes = [C.c_void_p, C.c_void_p, C.c_char_p, C.c_char_p, C.c_size_t]
+        err = C.create_string_buffer(512)
+        rc = self.L.pmh_msa_reroot(ctx.h, self.h, leaf_name.encode(), err, 512)
+        if rc:
+            raise PanmanError(rc, err.value.decode())
+        self._refresh()
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.L.pmh_build_free(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 class MsaPrepared:

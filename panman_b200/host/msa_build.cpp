@@ -34,6 +34,7 @@ struct pmh_build {
     std::vector<int64_t> tuple_off;
     std::vector<int32_t> tuple_pos;
     std::vector<uint8_t> tuple_tc;
+    bool ran = false;  // the lists above describe `tree` (pmh_msa_run / pmh_msa_reroot succeeded)
     double seconds[4] = {0, 0, 0, 0};
 };
 
@@ -210,6 +211,30 @@ std::string read_msa(const char* text, size_t len, bool strip_cr, std::map<std::
 
 pmh_build::~pmh_build() { pin_release(codes4, codes_cached); }
 
+namespace {
+// the lists of the pass just run on b->tree (pmb_result) and their run-merge (pmb_merge_runs) -> the build's NucMut fields
+void store_lists(pmh_build* b, const pmb_result& res, const pmb_nucmut_result& mr) {
+    const int32_t N = b->tree.t.n_nodes();
+    b->tuple_off.assign(res.node_offsets, res.node_offsets + N + 1);
+    b->tuple_pos.assign(res.pos, res.pos + res.n_mut);
+    b->tuple_tc.assign(res.type_code, res.type_code + res.n_mut);
+    b->nuc.assign(size_t(N), {});
+    for (int32_t v = 0; v < N; v++) {
+        const int64_t a = mr.node_offsets[v], z = mr.node_offsets[v + 1];
+        b->nuc[v].resize(size_t(z - a));
+        for (int64_t k = a; k < z; k++) {
+            pmh_nucmut& m = b->nuc[v][size_t(k - a)];
+            m.nucPosition = mr.nuc_position[k];
+            m.nucGapPosition = -1;
+            m.primaryBlockId = 0;
+            m.secondaryBlockId = -1;
+            m.mutInfo = mr.mut_info[k];
+            m.nucs = mr.nucs[k];
+        }
+    }
+}
+}  // namespace
+
 extern "C" {
 
 static pmh_tree* tree_from_newick_impl(const char* newick, char* err, size_t err_len) {
@@ -369,7 +394,10 @@ static int msa_run_impl(pmb_ctx* ctx, pmb_group* grp, pmh_build* b, char* err, s
     };
     const pmh::HostTree& T = b->tree.t;
     const int64_t n_cols = b->n_cols, stride = b->stride;
-    if (n_cols == 0) return PMB_OK;
+    if (n_cols == 0) {
+        b->ran = true;
+        return PMB_OK;
+    }
     const uint8_t* codes4 = b->codes4 ? b->codes4 : b->codes_pageable.data();
     if (!codes4 || b->present.empty()) return fail("the batch was already consumed by an earlier pmh_msa_run");
     const std::vector<uint8_t>& present = b->present;
@@ -398,26 +426,70 @@ static int msa_run_impl(pmb_ctx* ctx, pmb_group* grp, pmh_build* b, char* err, s
 
     // ---- lists are already per node in ascending position (= std::sort of the tuples, :1447); merge runs
     t0 = Clock::now();
-    b->tuple_off.assign(res.node_offsets, res.node_offsets + T.n_nodes() + 1);
-    b->tuple_pos.assign(res.pos, res.pos + res.n_mut);
-    b->tuple_tc.assign(res.type_code, res.type_code + res.n_mut);
     // greedy <= 6 run-merge on the device (pmb_merge_runs; src/panman.cpp:1445-1466, NucMut ctor src/panman.hpp:109-151)
     pmb_nucmut_result mr;
     rc = grp ? pmb_group_merge_runs(grp, /*to_host*/1, &mr) : pmb_merge_runs(ctx, /*source*/0, /*to_host*/1, &mr);
     if (rc) return fail(std::string("pmb_merge_runs: ") + engine_error());
-    for (int32_t v = 0; v < T.n_nodes(); v++) {
-        const int64_t a = mr.node_offsets[v], z = mr.node_offsets[v + 1];
-        b->nuc[v].resize(size_t(z - a));
-        for (int64_t k = a; k < z; k++) {
-            pmh_nucmut& m = b->nuc[v][size_t(k - a)];
-            m.nucPosition = mr.nuc_position[k];
-            m.nucGapPosition = -1;
-            m.primaryBlockId = 0;
-            m.secondaryBlockId = -1;
-            m.mutInfo = mr.mut_info[k];
-            m.nucs = mr.nucs[k];
-        }
+    store_lists(b, res, mr);
+    b->ran = true;
+    b->seconds[3] = since(t0);
+    return PMB_OK;
+}
+
+// Tree::reroot (reference src/reroot.cpp:4-261) of an MSA-built PanMAT: the tree is transformed (pmh::reroot_tree), every
+// leaf's sequence is rebuilt on the device from the build's Node::nucMutation (pmb_upload_replay: only the pieces cross the
+// link), and every column is inferred again by Fitch on the new tree with the root forced to the tip's own code
+// (src/reroot.cpp:134-224; also for a --low-mem-mode build), then run-merged (:226-261, the MSA form for one block).
+static int msa_reroot_impl(pmb_ctx* ctx, pmh_build* b, const char* leaf_name, char* err, size_t err_len) {
+    if (!ctx || !b || !leaf_name) { set_err(err, err_len, "null argument"); return PMB_ERR_INVALID; }
+    auto fail = [&](int rc, const std::string& m) -> int {
+        set_err(err, err_len, m);
+        return rc;
+    };
+    const pmh::HostTree& OT = b->tree.t;  // the tree the lists were built on
+    const int32_t tip = pmh::find_node(OT, leaf_name);
+    if (tip < 0) return fail(PMB_ERR_INVALID, std::string("Sequence with name ") + leaf_name + " not found!");  // src/reroot.cpp:5-8
+    if (!b->ran) return fail(PMB_ERR_NO_INPUT, "reroot works on a built PanMAT: call pmh_msa_run first");
+    pmh::HostTree nt;
+    const std::string e = pmh::reroot_tree(OT, tip, &nt);
+    if (!e.empty()) return fail(PMB_ERR_INVALID, e);
+    if (b->n_cols == 0) {
+        b->tree.t = std::move(nt);
+        b->nuc.assign(size_t(b->tree.t.n_nodes()), {});
+        b->tuple_off.assign(size_t(b->tree.t.n_nodes()) + 1, 0);
+        return PMB_OK;
     }
+    auto t0 = Clock::now();
+    const int32_t N = OT.n_nodes();
+    std::vector<int64_t> piece_off(size_t(N) + 1, 0);
+    for (int32_t v = 0; v < N; v++) piece_off[size_t(v) + 1] = piece_off[size_t(v)] + int64_t(b->nuc[size_t(v)].size());
+    std::vector<int32_t> pos(static_cast<size_t>(piece_off[size_t(N)]));
+    std::vector<uint8_t> info(pos.size());
+    std::vector<uint32_t> nucs(pos.size());
+    for (int32_t v = 0; v < N; v++)
+        for (size_t k = 0; k < b->nuc[size_t(v)].size(); k++) {
+            const pmh_nucmut& m = b->nuc[size_t(v)][k];
+            const size_t i = size_t(piece_off[size_t(v)]) + k;
+            pos[i] = m.nucPosition;
+            info[i] = m.mutInfo;
+            nucs[i] = m.nucs;
+        }
+    int rc = pmb_set_tree(ctx, nt.n_nodes(), nt.root, nt.child_off.data(), nt.child_idx.data(), nt.leaf_row.data());
+    if (rc) return fail(rc, std::string("pmb_set_tree: ") + pmb_last_error(ctx));
+    rc = pmb_upload_replay(ctx, N, OT.root, OT.child_off.data(), OT.child_idx.data(), OT.leaf_row.data(), piece_off.data(), pos.data(),
+                           info.data(), nucs.data(), b->n_cols, b->parent_code.data(), OT.leaf_row[tip]);
+    if (rc) return fail(rc, std::string("pmb_upload_replay: ") + pmb_last_error(ctx));
+    rc = pmb_run_resident(ctx, PMB_ALGO_FITCH, 0);
+    pmb_result res;
+    if (!rc) rc = pmb_download(ctx, &res);
+    if (rc) return fail(rc, std::string("pmb_run_resident: ") + pmb_last_error(ctx));
+    b->seconds[2] = since(t0);
+    t0 = Clock::now();
+    pmb_nucmut_result mr;
+    rc = pmb_merge_runs(ctx, /*source*/0, /*to_host*/1, &mr);
+    if (rc) return fail(rc, std::string("pmb_merge_runs: ") + pmb_last_error(ctx));
+    b->tree.t = std::move(nt);
+    store_lists(b, res, mr);
     b->seconds[3] = since(t0);
     return PMB_OK;
 }
@@ -471,6 +543,17 @@ int pmh_msa_run(pmb_ctx* ctx, pmh_build* b, char* err, size_t err_len) {
         return PMB_ERR_OOM;
     } catch (const std::exception& ex) {
         set_err(err, err_len, std::string("pmh_msa_run: ") + ex.what());
+        return PMB_ERR_INVALID;
+    }
+}
+int pmh_msa_reroot(pmb_ctx* ctx, pmh_build* b, const char* leaf_name, char* err, size_t err_len) {
+    try {
+        return msa_reroot_impl(ctx, b, leaf_name, err, err_len);
+    } catch (const std::bad_alloc&) {
+        set_err(err, err_len, "out of host memory");
+        return PMB_ERR_OOM;
+    } catch (const std::exception& ex) {
+        set_err(err, err_len, std::string("pmh_msa_reroot: ") + ex.what());
         return PMB_ERR_INVALID;
     }
 }

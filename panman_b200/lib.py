@@ -17,7 +17,7 @@ EXPORTS = ["pmb_create", "pmb_destroy", "pmb_last_error", "pmb_set_option", "pmb
            "pmb_group_upload_nuc", "pmb_group_upload_shard", "pmb_group_run_async", "pmb_group_wait",
            "pmb_group_result_device", "pmb_group_download", "pmb_group_merge_runs", "pmb_group_run_nuc",
            "pmb_runs_encode", "pmb_runs_free", "pmb_runs_describe", "pmb_upload_runs", "pmb_upload_runs_async", "pmb_run_runs",
-           "pmb_group_upload_runs", "pmb_group_upload_shard_runs", "pmb_group_run_runs", "pmb_join"]
+           "pmb_group_upload_runs", "pmb_group_upload_shard_runs", "pmb_group_run_runs", "pmb_join", "pmb_upload_replay"]
 GROUP_HANDLE_BYTES = 128
 
 
@@ -72,6 +72,7 @@ def load_library():
     L.pmb_set_tree.argtypes = [vp, i32, i32, vp, vp, vp]
     L.pmb_run_nuc.argtypes = [vp, C.c_int, i64, i32, vp, i64, vp, vp, vp, vp, i64, C.c_int, C.POINTER(pmb_result)]
     L.pmb_upload_nuc.argtypes = [vp, i64, i32, vp, i64, vp, vp, vp, vp, i64]
+    L.pmb_upload_replay.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, i64, vp, i32]
     L.pmb_run_resident.argtypes = [vp, C.c_int, C.c_int]
     L.pmb_run_resident_async.argtypes = [vp, C.c_int, C.c_int]
     L.pmb_wait.argtypes = [vp]
