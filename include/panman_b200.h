@@ -294,7 +294,8 @@ int pmb_group_connect(pmb_group* group, const void* all_handles /* world x PMB_G
 /* Inputs. pmb_group_upload_nuc takes the WHOLE alignment (arguments as pmb_upload_nuc, positions count from column 0):
  * every local rank copies its own column range out of it. pmb_group_upload_shard takes one local rank's range only (the
  * caller sliced or generated it): column col_begin of the range is the low nibble of byte 0 of every row, parent_code /
- * root_override / fwd_root_ref start at col_begin too. Uploads of the local ranks run concurrently. */
+ * root_override / fwd_root_ref start at col_begin too. Uploads of the local ranks run concurrently. pmb_group_upload_nuc
+ * refuses row_stride_bytes < (n_cols + 1) / 2 (PMB_ERR_INVALID): the stride is that of the whole row, not of a range. */
 int pmb_group_upload_nuc(pmb_group* group, int64_t n_cols, int32_t n_rows, const uint8_t* leaf_codes_4bit, int64_t row_stride_bytes,
                          const uint8_t* leaf_present, const uint8_t* parent_code, const int8_t* root_override,
                          const int8_t* fwd_root_ref);

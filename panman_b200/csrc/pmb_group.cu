@@ -241,7 +241,9 @@ int enqueue_step(pmb_group* g, int algo, int flags, uint32_t s) {
         for (int r = 0; r < g->active; r++) G_CU(g->wait32(ms, CUdeviceptr(l0.box + BOX_ARRIVE + 4 * size_t(r)), s, CU_STREAM_WAIT_VALUE_GEQ));
         int rc = pmb_merge_packed(l0.ctx, g->active, l0.box + BOX_SLOTS + buf, g->capacity, g->merge_stream, &g->merged);
         if (rc) return gctx(g, rc, l0);
-        for (int r = 0; r < g->active; r++) G_CU(g->write32(ms, CUdeviceptr(g->peer_box[size_t(r)] + BOX_CREDIT), s, CU_STREAM_WRITE_VALUE_DEFAULT));
+        // every rank's box, the ranks that sat this step out included: a rank that was inactive for two or more steps (or since
+        // the reserve) and becomes active with a wider alignment waits for credit >= s - 2, which only this write can satisfy
+        for (int r = 0; r < g->world; r++) G_CU(g->write32(ms, CUdeviceptr(g->peer_box[size_t(r)] + BOX_CREDIT), s, CU_STREAM_WRITE_VALUE_DEFAULT));
         g->have_merged = true;
     }
     return PMB_OK;
@@ -256,7 +258,7 @@ void unblock_step(pmb_group* g, uint32_t s) {
         if (cudaStreamCreateWithFlags(&aux, cudaStreamNonBlocking) != cudaSuccess) continue;
         g->write32(static_cast<CUstream>(aux), CUdeviceptr(l.root_box + BOX_ARRIVE + 4 * size_t(g->rank_base + i)), s, CU_STREAM_WRITE_VALUE_DEFAULT);
         if (g->has_root())
-            for (int r = 0; r < g->active && r < int(g->peer_box.size()); r++)
+            for (int r = 0; r < int(g->peer_box.size()); r++)  // every rank, as enqueue_step
                 if (g->peer_box[size_t(r)]) g->write32(static_cast<CUstream>(aux), CUdeviceptr(g->peer_box[size_t(r)] + BOX_CREDIT), s, CU_STREAM_WRITE_VALUE_DEFAULT);
         cudaStreamSynchronize(aux);
         cudaStreamDestroy(aux);
@@ -532,6 +534,9 @@ int pmb_group_upload_nuc(pmb_group* g, int64_t n_cols, int32_t n_rows, const uin
                          const uint8_t* leaf_present, const uint8_t* parent_code, const int8_t* root_override,
                          const int8_t* fwd_root_ref) {
     if (!g || n_cols <= 0 || !leaf_codes_4bit || !parent_code) return g ? gfail(g, PMB_ERR_INVALID, "bad input arguments") : PMB_ERR_INVALID;
+    // each rank's upload checks the stride against its own range only: a stride too small for the whole row would pass there
+    // and make the ranks past 0 read overlapping rows
+    if (row_stride_bytes < (n_cols + 1) / 2) return gfail(g, PMB_ERR_INVALID, "row_stride_bytes too small for n_cols");
     for (int i = 0; i < g->n_local; i++) {
         int64_t b, e;
         range_of(g->world, n_cols, g->rank_base + i, &b, &e);  // b is a multiple of 1024: a whole byte of every row
